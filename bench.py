@@ -2,7 +2,7 @@
 """bench.py -- pdgstrf3d factorization GFlop/s (FP64) of the B200-native path, with its roofline,
 end-to-end (host buffers) figure and the reference's CPU path timed beside it.
 
-    python bench.py [--gpus N --steps K --warmup W] [--grid G] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--grid G] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one numeric factorization (pdgstrf3d) of the 3D 7-point Poisson matrix on a G^3 grid
 (BASELINE.json configs[1] shape; geometric nested dissection as MY_PERMC, NOROWPERM, no
@@ -36,6 +36,7 @@ import numpy as np  # noqa: E402
 
 METRIC = "pdgstrf3d_factor_gflops_fp64"
 UNIT = "GFlop/s"
+DUMP_SAMPLE = 3_000_000     # --dump-outputs: values per factor arena, so that the two float64 samples stay under 64 MB
 
 
 
@@ -87,7 +88,12 @@ def parse():
                          "slu_b200_solve (no host copy of L/U at all: the mode of the largest runs); e2e is not measured")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-phases", type=int, default=1)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the L and U factors of the last one to DIR/*.npy (float64; a fixed, "
+                         f"seeded sample of each arena larger than {DUMP_SAMPLE:,} values), to compare two builds")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.grid <= 0:
         a.grid = 68 if a.workload == "fem3" else 128
     if a.cpu_grid <= 0:
@@ -320,6 +326,17 @@ def dgemm_peak_tflops(torch, m=8192, n=8192, k=256, reps=10):
     return 2.0 * m * n * k / best * 1e-9
 
 
+def dump_outputs(path, layer, suffix=""):
+    """The factors a caller of the timed path receives (L and U arenas of one layer) as float64 .npy files.  Arenas
+    larger than DUMP_SAMPLE are sampled at sorted positions drawn from a fixed seed, so that the same arguments select
+    the same entries in every run and two builds can be compared entry for entry."""
+    os.makedirs(path, exist_ok=True)
+    rng = np.random.default_rng(0)
+    for name, arena in (("L", layer.lval), ("U", layer.uval)):
+        pos = np.sort(rng.choice(arena.size, DUMP_SAMPLE, replace=False)) if arena.size > DUMP_SAMPLE else slice(None)
+        np.save(os.path.join(path, f"{name}{suffix}.npy"), np.asarray(arena[pos], np.float64))
+
+
 def main():
     args = parse()
     if args.impl == "reference":
@@ -417,6 +434,9 @@ def main():
     sampler.start()
     step_s = [allmax(one_step()) for _ in range(args.steps)]
     clocks = sampler.stop()
+    if args.dump_outputs:
+        h.download()                     # the factors of the last timed step, into the host arrays (refilled below)
+        dump_outputs(args.dump_outputs, lay, f"_rank{rank}" if world > 1 else "")
     st = h.stats()
     total_ops = allsum(st.ops_fact)
     t_step = float(np.mean(step_s))

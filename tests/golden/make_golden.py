@@ -1,6 +1,6 @@
 """Generate the golden fixtures of tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container (needs /root/reference and `make -C oracle ref`):
+Needs the reference binaries under oracle/_ref (`make -C oracle ref REF=<SuperLU_DIST source tree>`):
 
     python tests/golden/make_golden.py
 
@@ -8,7 +8,9 @@ Each fixture is the input of pdgstrf3d (dLUstruct_t + dtrf3Dpartition_t as the r
 and the factors the reference's own pdgstrf3d (CPU path, 1x1x1, OMP_NUM_THREADS=1, scipy OpenBLAS)
 produced, captured by the hook oracle/ref_build/pdgstrf3d_hook.c (SLU_B200_HOOK=dump).
 """
+import gzip
 import os
+import shutil
 import subprocess
 import sys
 import tempfile
@@ -18,7 +20,6 @@ sys.path.insert(0, ROOT)
 from superlu_dist_b200 import dumpio, hostlib, matgen  # noqa: E402
 
 REF = os.path.join(ROOT, "oracle", "_ref")
-EX = "/root/reference/EXAMPLE"
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -30,21 +31,25 @@ def run(cmd, dump):
 
 def main():
     with tempfile.TemporaryDirectory() as tmp:
+        # the reference's EXAMPLE matrices are stored here gzipped; the drivers read them unpacked
+        for f in ("g4.rua", "g20.rua", "cg20.cua"):
+            with gzip.open(os.path.join(OUT, f + ".gz"), "rb") as src, open(os.path.join(tmp, f), "wb") as dst:
+                shutil.copyfileobj(src, dst)
         # config #1 of BASELINE.json: EXAMPLE/pddrive3d on g20.rua, 1x1x1 (default options:
         # equilibration, MC64 row permutation, MMD(A'+A) column ordering)
         for name in ("g4", "g20"):
             pre, post = run([os.path.join(REF, "pddrive3d"), "-r", "1", "-c", "1", "-d", "1",
-                             os.path.join(EX, name + ".rua")], os.path.join(tmp, name))
+                             os.path.join(tmp, name + ".rua")], os.path.join(tmp, name))
             dumpio.save_npz(os.path.join(OUT, name + "_pddrive3d.npz"), pre, post)
         # config #5 of BASELINE.json (doublecomplex mirror): pzdrive3d on cg20.cua, and the same file with every
         # value scaled by 1000 ("cg20.cua scaled x1000", reading B of SURVEY 8d: exercises anorm/thresh scaling)
-        pre, post = run([os.path.join(REF, "pzdrive3d"), "-r", "1", "-c", "1", "-d", "1", os.path.join(EX, "cg20.cua")],
+        pre, post = run([os.path.join(REF, "pzdrive3d"), "-r", "1", "-c", "1", "-d", "1", os.path.join(tmp, "cg20.cua")],
                         os.path.join(tmp, "cg20"))
         dumpio.save_npz(os.path.join(OUT, "cg20_pzdrive3d.npz"), pre, post)
         # same matrix, tiny-pivot replacement on, no row permutation, smaller supernodes
         mat = os.path.join(tmp, "p.bin")
         for tag, N, leaf, extra in (("poisson8_nd", 8, 8, ["--maxsup", "16", "--relax", "4"]),
-                                    ("poisson12_nd_tiny", 12, 16, ["--maxsup", "24", "--relax", "6", "--tiny", "1"])):
+                                    ("poisson9_nd_tiny", 9, 16, ["--maxsup", "24", "--relax", "6", "--tiny", "1"])):
             rp, ci, v = hostlib.poisson3d(N)
             matgen.write_matrix_bin(mat, rp, ci, v)
             perm = hostlib.nd_order(N, leaf=leaf)

@@ -10,6 +10,8 @@ import sys
 
 import pytest
 
+from test_dropin import ZDRV
+
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -48,6 +50,7 @@ def test_diag_lu_cluster():
     _run("diagcluster")
 
 
+@pytest.mark.skipif(not os.path.exists(ZDRV), reason="oracle/_ref/pzdrive3d (the reference's own driver) not built")
 def test_optin_pzdrive3d_dropin():
     _run("zdropin")
 

@@ -1,6 +1,7 @@
 """Matrix-file readers of libslu_b200_host (SURVEY 8f N4): Harwell-Boeing, Matrix Market, the reference's binary dump.
 Checked against SciPy's independent readers/writers on generated matrices, and against the reference's own EXAMPLE
-fixtures where /root/reference exists (this container; skipped on the GPU box)."""
+fixtures (g4.rua, g20.rua, big.rua, cg20.cua, stored gzipped and otherwise unchanged in tests/golden)."""
+import gzip
 import os
 
 import numpy as np
@@ -10,7 +11,7 @@ import scipy.sparse as sp
 
 from superlu_dist_b200 import hostlib, matgen
 
-REF_EX = "/root/reference/EXAMPLE"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _rand(n, density, seed, sym=False, cx=False):
@@ -126,10 +127,11 @@ def test_errors(tmp_path):
         hostlib.read_matrix(str(tmp_path / "bad.mtx"))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_EX), reason="the reference's EXAMPLE fixtures exist only where /root/reference does")
 @pytest.mark.parametrize("name", ["g4.rua", "g20.rua", "big.rua", "cg20.cua"])
-def test_reference_fixtures(name):
-    nr, nc, ptr, ind, val = hostlib.read_matrix(os.path.join(REF_EX, name))
+def test_reference_fixtures(tmp_path, name):
+    with gzip.open(os.path.join(GOLDEN, name + ".gz"), "rb") as f:
+        (tmp_path / name).write_bytes(f.read())
+    nr, nc, ptr, ind, val = hostlib.read_matrix(str(tmp_path / name))
     a = _as_csr(nr, nc, ptr, ind, val)
     expect = {"g4.rua": (16, 64), "g20.rua": (400, 1920), "big.rua": (4960, 23884), "cg20.cua": (400, 1920)}[name]
     assert (nr, a.nnz) == expect
