@@ -114,12 +114,13 @@ typedef struct {
                                   /* only filled when options.verbose >= 2 (adds syncs)      */
     int64_t lu_device_bytes;      /* HBM held by L/U values                                  */
     int64_t index_device_bytes;   /* HBM held by index structures + workspace                */
-    int64_t nnz_l, nnz_u;         /* doubles stored in my L / U panels (device layout)       */
+    int64_t nnz_l, nnz_u;         /* elements (complex: pairs) in my L / U panels (device)   */
     int32_t nlevels;              /* level-synchronous steps executed                        */
     int32_t my_supernodes;        /* supernodes this rank factored                           */
     double reserved[8];           /* [0] ms spent slicing (verbose >= 2), [1] Schur flops taken by the */
                                   /* tcgen05 path, [2] bytes of its int8 workspace, [3] slices in use,  */
-                                  /* [4] seconds of the last slu_b200_solve, [5] its kernel launches    */
+                                  /* [4] seconds of the last slu_b200_solve / slu_b200_z_solve,         */
+                                  /* [5] its kernel launches                                            */
 } slu_b200_stats_t;
 
 typedef struct slu_b200_handle_s *slu_b200_handle_t;
@@ -222,6 +223,14 @@ int slu_b200_z_plan(const slu_b200_lu_view_t *lu, const slu_b200_options_t *opt,
 void slu_b200_z_destroy(slu_b200_zhandle_t h);
 /* drop-in body of pzgstrf3d (complex16/pzgstrf3d.c:120-123): create + upload + factor + download + destroy */
 int pzgstrf3d_b200(const slu_b200_lu_view_t *lu, const slu_b200_options_t *opt, slu_b200_stats_t *stats, int *info);
+/* Device-side distribution, as slu_b200_fill_csr (the job of pzdistribute3d, SRC/complex16/pzdistribute3d.c:24):
+ * val holds nnz (re, im) pairs; 20 bytes per nonzero cross PCIe instead of 16 bytes per factor entry.  1 x 1 x Pz. */
+int slu_b200_z_fill_csr(slu_b200_zhandle_t h, int n, const int32_t *rowptr, const int32_t *colind,
+                        const double *val, const int32_t *perm);
+/* Solve L U x = b on the resident factors, as slu_b200_solve (the job of pzgstrs3d, SRC/complex16/pzgstrs3d.c:6694):
+ * x holds n x nrhs (re, im) pairs column-major, ldx counts complex elements.  1 x 1 x Pz grids: collective, every rank
+ * passes the same b and receives the full x.  stats.reserved[4] = seconds of the call, [5] = its kernel launches. */
+int slu_b200_z_solve(slu_b200_zhandle_t h, double *x, int ldx, int nrhs);
 void slu_b200_z_comm_cache_clear(void);   /* called by slu_b200_comm_cache_clear */
 /* kernel-level test entries; arrays are interleaved (re, im), sizes in complex elements */
 int slu_b200_z_k_diag_lu(double *a, int ns, int lda, int replace_tiny, double thresh, int col0, int *info, int *tiny);

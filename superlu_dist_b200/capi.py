@@ -96,6 +96,8 @@ def lib():
     L.slu_b200_z_factor.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
     L.slu_b200_z_factor_host.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
     L.slu_b200_z_get_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
+    L.slu_b200_z_solve.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
+    L.slu_b200_z_fill_csr.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.slu_b200_z_destroy.argtypes = [C.c_void_p]
     L.slu_b200_z_destroy.restype = None
     L.pzgstrf3d_b200.argtypes = [C.POINTER(LUView), C.POINTER(Options), C.POINTER(Stats), C.POINTER(C.c_int)]
@@ -264,23 +266,24 @@ class Handle:
         _check(_fn("download", self.z_)(self.h))
 
     def fill_csr(self, rowptr, colind, val, perm):
-        """Device-side distribution (slu_b200_fill_csr): P A P^T scattered into the HBM panels by a kernel; replaces
-        upload().  perm[old] = new."""
+        """Device-side distribution (slu_b200_fill_csr / slu_b200_z_fill_csr): P A P^T scattered into the HBM panels by
+        a kernel; replaces upload().  perm[old] = new; val is complex128 for a complex handle."""
         rp = np.ascontiguousarray(rowptr, np.int32)
         ci = np.ascontiguousarray(colind, np.int32)
-        v = np.ascontiguousarray(val, np.float64)
+        if self.z_:
+            v = np.ascontiguousarray(val, np.complex128).view(np.float64)
+        else:
+            v = np.ascontiguousarray(val, np.float64)
         pm = np.ascontiguousarray(perm, np.int32)
-        _check(lib().slu_b200_fill_csr(self.h, len(rp) - 1, rp.ctypes.data_as(C.c_void_p), ci.ctypes.data_as(C.c_void_p),
-                                       v.ctypes.data_as(C.c_void_p), pm.ctypes.data_as(C.c_void_p)))
+        _check(_fn("fill_csr", self.z_)(self.h, len(rp) - 1, rp.ctypes.data_as(C.c_void_p), ci.ctypes.data_as(C.c_void_p),
+                                        v.ctypes.data_as(C.c_void_p), pm.ctypes.data_as(C.c_void_p)))
 
     def solve(self, b):
-        """L U x = b on the device-resident factors (slu_b200_solve); b: (n,) or (nrhs, n), ordering of the factored
-        matrix.  Returns x with the same shape."""
-        if self.z_:
-            raise TypeError("slu_b200_solve is implemented for the double path")
-        x = np.array(b, np.float64, order="C", copy=True)
+        """L U x = b on the device-resident factors (slu_b200_solve / slu_b200_z_solve); b: (n,) or (nrhs, n), ordering
+        of the factored matrix, complex128 for a complex handle.  Returns x with the same shape."""
+        x = np.array(b, np.complex128 if self.z_ else np.float64, order="C", copy=True)
         nrhs = 1 if x.ndim == 1 else x.shape[0]
-        _check(lib().slu_b200_solve(self.h, x.ctypes.data_as(C.c_void_p), self.prob.n, nrhs))
+        _check(_fn("solve", self.z_)(self.h, x.ctypes.data_as(C.c_void_p), self.prob.n, nrhs))
         return x
 
     def stats(self):

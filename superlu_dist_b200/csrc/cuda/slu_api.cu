@@ -30,6 +30,8 @@
 #define slu_b200_get_stats slu_b200_z_get_stats
 #define slu_b200_destroy slu_b200_z_destroy
 #define slu_b200_plan slu_b200_z_plan
+#define slu_b200_solve slu_b200_z_solve
+#define slu_b200_fill_csr slu_b200_z_fill_csr
 #define pdgstrf3d_b200 pzgstrf3d_b200
 #define slu_b200_k_diag_lu slu_b200_z_k_diag_lu
 #define slu_b200_k_trsm_l slu_b200_z_k_trsm_l
@@ -230,7 +232,7 @@ struct slu_b200_handle_s {
     int tc_slices = 0, tc_min_ns = 0;     // 0 slices: tcgen05 path off
     bool tc_force_off = false, tc_alloc_failed = false;   // slice workspace did not fit: analysed again without the tcgen05 path
     int tc_nonatomic = 0;                 // plain load/store scatter for destinations only one supernode of a level updates
-    DevBuf<double> d_x, d_x2;             // triangular solve: right-hand sides / solution
+    DevBuf<val_t> d_x, d_x2;              // triangular solve: right-hand sides / solution
     std::vector<int64_t> z_nodes_off;     // [zl] offset into d_pool_i32 of the forest's node list (solve masks)
     bool factored = false;
     DevBuf<int> d_flags;                  // [0]=info [1]=err
@@ -1592,11 +1594,12 @@ int slu_b200_factor_host(slu_b200_handle_t H, int *info)
     return rc;
 }
 
-#ifndef SLU_COMPLEX
 // Device-side distribution (SURVEY 8f row N1): A arrives as host CSR (the caller's matrix, perm[old] = new as
 // ScalePermstruct->perm_c after sp_colorder), is copied to HBM once (12 bytes per nonzero instead of 8 bytes per FACTOR
-// entry) and scattered into the panels by a kernel -- what pddistribute3d does on the host.  Replicated ancestors of
-// other layers start at zero (dinit3DLUstructForest, pdgssvx3d.c:948).  Replaces slu_b200_upload.
+// entry; 20 instead of 16 in doublecomplex) and scattered into the panels by a kernel -- what pddistribute3d /
+// pzdistribute3d (SRC/complex16/pzdistribute3d.c:24) do on the host.  Replicated ancestors of other layers start at
+// zero (dinit3DLUstructForest, pdgssvx3d.c:948).  Replaces slu_b200_upload.  Both precisions: val holds nnz elements of
+// val_t ((re, im) pairs in doublecomplex).
 int slu_b200_fill_csr(slu_b200_handle_t H, int n, const int32_t *rowptr, const int32_t *colind, const double *val, const int32_t *perm)
 {
     if (!H || !rowptr || !colind || !val || !perm) return fail("null argument");
@@ -1605,7 +1608,7 @@ int slu_b200_fill_csr(slu_b200_handle_t H, int n, const int32_t *rowptr, const i
     double t0 = now_s();
     const int64_t nnz = rowptr[n];
     DevBuf<int32_t> drp, dci, dperm;
-    DevBuf<double> dv;
+    DevBuf<val_t> dv;
     DevBuf<int8_t> dact;
     std::vector<int8_t> act(H->nsupers, 0);
     for (int zl = 0; zl < H->max_lvl; ++zl)
@@ -1615,7 +1618,7 @@ int slu_b200_fill_csr(slu_b200_handle_t H, int n, const int32_t *rowptr, const i
     cudaStream_t s = H->stream;
     CU(cudaMemcpyAsync(drp.p, rowptr, ((size_t)n + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(dci.p, colind, (size_t)nnz * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    CU(cudaMemcpyAsync(dv.p, val, (size_t)nnz * sizeof(double), cudaMemcpyHostToDevice, s));
+    CU(cudaMemcpyAsync(dv.p, val, (size_t)nnz * sizeof(val_t), cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(dperm.p, perm, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     CU(cudaMemsetAsync(H->val.p, 0, H->val.bytes(), s));
     CU(cudaMemsetAsync(H->d_flags.p + 1, 0, sizeof(int), s));
@@ -1631,11 +1634,12 @@ int slu_b200_fill_csr(slu_b200_handle_t H, int n, const int32_t *rowptr, const i
     return 0;
 }
 
-// Triangular solves on the resident factors (the job of pdgstrs3d, SRC/double/pdgstrs3d.c:6604, for factors that never
-// left HBM).  Along Z: forward, the partial vectors climb the Z tree -- an all-reduce over the group of each level,
-// after which only the group's owner layer keeps the vector (the reference reduces the ancestor contributions
-// pairwise); backward, the owner's solution is spread to its group the same way (dbroadcastAncestor3d,
-// pd3dcomm.c:1145); a last all-reduce of the owned pieces gives every rank the full solution.
+// Triangular solves on the resident factors (the job of pdgstrs3d, SRC/double/pdgstrs3d.c:6604, and of pzgstrs3d,
+// SRC/complex16/pzgstrs3d.c:6694, for factors that never left HBM); xh holds n x nrhs elements of val_t.  Along Z:
+// forward, the partial vectors climb the Z tree -- an all-reduce over the group of each level, after which only the
+// group's owner layer keeps the vector (the reference reduces the ancestor contributions pairwise); backward, the
+// owner's solution is spread to its group the same way (dbroadcastAncestor3d, pd3dcomm.c:1145); a last all-reduce of
+// the owned pieces gives every rank the full solution.
 int slu_b200_solve(slu_b200_handle_t H, double *xh, int ldx, int nrhs)
 {
     if (!H || !xh) return fail("null argument");
@@ -1648,27 +1652,27 @@ int slu_b200_solve(slu_b200_handle_t H, double *xh, int ldx, int nrhs)
     if (H->d_x.n < len && (H->d_x.alloc(len) || H->d_x2.alloc(len))) return -1;
     cudaStream_t s = H->stream;
     const DeviceLU &d = H->dev;
-    double *x = H->d_x.p, *x2 = H->d_x2.p;
+    val_t *x = H->d_x.p, *x2 = H->d_x2.p;
     double t0 = now_s();
-    CU(cudaMemcpy2DAsync(x2, (size_t)n * sizeof(double), xh, (size_t)ldx * sizeof(double), (size_t)n * sizeof(double), (size_t)nrhs,
+    CU(cudaMemcpy2DAsync(x2, (size_t)n * sizeof(val_t), xh, (size_t)ldx * sizeof(val_t), (size_t)n * sizeof(val_t), (size_t)nrhs,
                          cudaMemcpyHostToDevice, s));
     const bool multi = H->comm != nullptr;
     int launches = 0;
     auto forest_nodes = [&](int zl) { return H->d_pool_i32.p + H->z_nodes_off[zl]; };
     if (multi) {      // start from the entries this rank owns: b on the owner layer of every forest, 0 elsewhere
-        CU(cudaMemsetAsync(x, 0, len * sizeof(double), s));
+        CU(cudaMemsetAsync(x, 0, len * sizeof(val_t), s));
         for (int zl = 0; zl < H->max_lvl; ++zl)
             if (!H->my_zero[zl]) launches += launch_solve_mask(d, forest_nodes(zl), (int)H->znodes[zl].size(), x, n, nrhs, x2, s);
     } else {
-        CU(cudaMemcpyAsync(x, x2, len * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        CU(cudaMemcpyAsync(x, x2, len * sizeof(val_t), cudaMemcpyDeviceToDevice, s));
     }
     const int64_t *p64 = H->d_pool_i64.p;
     // forward: L y = b
     size_t li = 0;
     for (int zl = 0; zl < H->max_lvl; ++zl) {
         if (multi && zl >= 1) {
-            NC(g_nccl.AllReduce(x, x, len, NCCL_FLOAT64, NCCL_SUM, H->gcomm[zl], s));
-            if (H->my_zero[zl]) CU(cudaMemsetAsync(x, 0, len * sizeof(double), s));
+            NC(g_nccl.AllReduce(x, x, len * VAL_DOUBLES, NCCL_FLOAT64, NCCL_SUM, H->gcomm[zl], s));
+            if (H->my_zero[zl]) CU(cudaMemsetAsync(x, 0, len * sizeof(val_t), s));
         }
         for (; li < H->levels.size() && H->levels[li].zlvl <= zl; ++li) {
             const LevelPlan &L = H->levels[li];
@@ -1693,19 +1697,19 @@ int slu_b200_solve(slu_b200_handle_t H, double *xh, int ldx, int nrhs)
             }
         li = lo;
         if (multi && zl >= 1) {
-            if (H->my_zero[zl]) CU(cudaMemsetAsync(x, 0, len * sizeof(double), s));
-            NC(g_nccl.AllReduce(x, x, len, NCCL_FLOAT64, NCCL_SUM, H->gcomm[zl], s));
+            if (H->my_zero[zl]) CU(cudaMemsetAsync(x, 0, len * sizeof(val_t), s));
+            NC(g_nccl.AllReduce(x, x, len * VAL_DOUBLES, NCCL_FLOAT64, NCCL_SUM, H->gcomm[zl], s));
         }
     }
-    double *result = x;
+    val_t *result = x;
     if (multi) {      // every rank contributes the entries it owns: the full solution everywhere
-        CU(cudaMemsetAsync(x2, 0, len * sizeof(double), s));
+        CU(cudaMemsetAsync(x2, 0, len * sizeof(val_t), s));
         for (int zl = 0; zl < H->max_lvl; ++zl)
             if (!H->my_zero[zl]) launches += launch_solve_mask(d, forest_nodes(zl), (int)H->znodes[zl].size(), x2, n, nrhs, x, s);
-        NC(g_nccl.AllReduce(x2, x2, len, NCCL_FLOAT64, NCCL_SUM, H->comm, s));
+        NC(g_nccl.AllReduce(x2, x2, len * VAL_DOUBLES, NCCL_FLOAT64, NCCL_SUM, H->comm, s));
         result = x2;
     }
-    CU(cudaMemcpy2DAsync(xh, (size_t)ldx * sizeof(double), result, (size_t)n * sizeof(double), (size_t)n * sizeof(double), (size_t)nrhs,
+    CU(cudaMemcpy2DAsync(xh, (size_t)ldx * sizeof(val_t), result, (size_t)n * sizeof(val_t), (size_t)n * sizeof(val_t), (size_t)nrhs,
                          cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     CU(cudaGetLastError());
@@ -1713,7 +1717,6 @@ int slu_b200_solve(slu_b200_handle_t H, double *xh, int ldx, int nrhs)
     H->st.reserved[5] = (double)launches;
     return 0;
 }
-#endif
 
 #ifndef SLU_COMPLEX
 // ---- benchmark support (SURVEY 8a row a10: the reference's GPU Schur path is "to be beaten") ------------------------

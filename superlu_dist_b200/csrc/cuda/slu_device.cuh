@@ -148,16 +148,18 @@ struct UpSeg { int64_t dst, src, len; };  // a transfer chunk: arena offset, (un
 int launch_gemm_sub(int m, int n, int k, const val_t *a, int lda, const val_t *b, int ldb, val_t *c,
                     int ldc, int variant, cudaStream_t s);
 
-#ifndef SLU_COMPLEX
-// slu_solve.cu: triangular solves on the resident factors.  x: device, n x nrhs, ordering of the factored matrix
+// slu_solve.cu / slu_solve_z.cu: triangular solves on the resident factors.  x: device, n x nrhs, ordering of the
+// factored matrix
 constexpr int SOLVE_TILE = 256;
-int launch_solve_diag(const DeviceLU &d, const int32_t *nodes, int count, bool upper, double *x, int n, int nrhs, cudaStream_t s);
-int launch_solve_update(const DeviceLU &d, const Batch &b, int64_t ctas, bool upper, double *x, int n, int nrhs, cudaStream_t s);
+int launch_solve_diag(const DeviceLU &d, const int32_t *nodes, int count, bool upper, val_t *x, int n, int nrhs, cudaStream_t s);
+int launch_solve_update(const DeviceLU &d, const Batch &b, int64_t ctas, bool upper, val_t *x, int n, int nrhs, cudaStream_t s);
 // x[entries of the listed supernodes] = src[...] (src == nullptr: 0)
-int launch_solve_mask(const DeviceLU &d, const int32_t *nodes, int count, double *x, int n, int nrhs, const double *src, cudaStream_t s);
+int launch_solve_mask(const DeviceLU &d, const int32_t *nodes, int count, val_t *x, int n, int nrhs, const val_t *src, cudaStream_t s);
 // device-side distribution of a CSR matrix (device arrays) into the arena; *err counts entries without a slot
-int launch_fill_csr(const DeviceLU &d, int n, const int32_t *rowptr, const int32_t *colind, const double *aval, const int32_t *perm,
+int launch_fill_csr(const DeviceLU &d, int n, const int32_t *rowptr, const int32_t *colind, const val_t *aval, const int32_t *perm,
                     const int8_t *active, int *err, cudaStream_t s);
+
+#ifndef SLU_COMPLEX
 // slu_ozaki.cu: the Schur update of wide supernodes on tcgen05 (int8 slices, exact int32 accumulation in TMEM)
 constexpr int OZ_NT = 32;             // columns of one CTA's tcgen05 Schur tile (rows: 128)
 constexpr int OZ_CL = 1;              // CTAs per cluster sharing the A operand by multicast (2 and 4 measured SLOWER: r02_notes.md)
